@@ -27,6 +27,10 @@ One JSON line is printed by rank 0:
   cpu_baseline the CPU oracle port (oracle/shards.py, torch fp32 on the host cores) on a bounded sample
 `--impl reference` times that CPU port as the reference arm with the same thread calibration and the same `config`
 (the reference is Python and cannot travel to the GPU box; see DESIGN.md).
+
+`--steps K` is the number of timed micro-batches in every arm. `--dump-outputs DIR` writes what the timed path returned
+for its last micro-batch (the logits) as `DIR/<name>.npy` in float32: inputs and weights are seeded, so two builds run
+with the same arguments can be compared output for output.
 """
 import argparse
 import faulthandler
@@ -38,6 +42,7 @@ import sys
 import threading
 import time
 
+import numpy as np
 import torch
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
@@ -54,6 +59,18 @@ WORKLOADS = {
     'vit-base-b1': ('google/vit-base-patch16-224', 1, 0, 0, 'images/sec per pipeline', 'images/s'),   # BASELINE configs[0]
 }
 N_INPUTS = 16   # distinct resident micro-batches the timed loop rotates over
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_output(out_dir: str, name: str, t: torch.Tensor) -> None:
+    """Write `t` as `out_dir/<name>.npy` in float32. Beyond DUMP_LIMIT_BYTES only a fixed, seeded sample of its rows is
+    written (the same rows in every run)."""
+    os.makedirs(out_dir, exist_ok=True)
+    a = t.detach().float().cpu()
+    if a.numel() * 4 > DUMP_LIMIT_BYTES:
+        rows = max(1, DUMP_LIMIT_BYTES // (4 * a[0].numel()))
+        a = a[torch.randperm(a.shape[0], generator=torch.Generator().manual_seed(0))[:rows].sort().values]
+    np.save(os.path.join(out_dir, f'{name}.npy'), a.numpy())
 
 
 def even_partition(layers: int, n: int):
@@ -212,8 +229,8 @@ def cpu_forward_timer(spec, ubatch: int, seq: int):
                                               'median_s_by_threads': {str(k): round(v, 4) for k, v in log.items()}}
 
 
-def cpu_sample(spec, ubatch: int, seq: int, unit: str, max_steps: int, budget_s: float) -> dict:
-    """Time the CPU port on a bounded sample; the same routine serves `cpu_baseline` and `--impl reference`."""
+def cpu_sample(spec, ubatch: int, seq: int, unit: str, steps: int) -> dict:
+    """Time `steps` forwards of the CPU port; the same routine serves `cpu_baseline` and `--impl reference`."""
     fwd, cores, cal = cpu_forward_timer(spec, ubatch, seq)
     # Warm-up until the per-forward time has settled: the first forwards of a process run ~2x slower than its steady state
     # (the allocator still maps and unmaps the 10-100 MB temporaries of every layer; r02g: 0.31 s vs 0.14 s per
@@ -230,14 +247,12 @@ def cpu_sample(spec, ubatch: int, seq: int, unit: str, max_steps: int, budget_s:
         last = min(last, dt1)
     cal['warmup_forwards'] = warm
     t0 = time.perf_counter()
-    n = 0
-    while n < 2 or (n < max_steps and time.perf_counter() - t0 < budget_s):
-        fwd()
-        n += 1
+    for _ in range(steps):
+        logits = fwd()
     dt = time.perf_counter() - t0
-    return {'value': n * ubatch / dt, 'unit': unit, 'cores': cores, 'kind': 'port', 'steps': n, 'seconds': dt,
-            'calibration': cal,
-            'sample': f"{n} micro-batches of {ubatch} through all {spec.layers} sub-layers, torch fp32 CPU "
+    return {'value': steps * ubatch / dt, 'unit': unit, 'cores': cores, 'kind': 'port', 'steps': steps, 'seconds': dt,
+            'calibration': cal, 'logits': logits,
+            'sample': f"{steps} micro-batches of {ubatch} through all {spec.layers} sub-layers, torch fp32 CPU "
                       f"({dt:.1f} s), 1 process x {cores} threads of {cal['host_cores']} usable host cores "
                       "(median-of-3 thread calibration)"}
 
@@ -277,7 +292,9 @@ def run_reference_arm(args, spec, ubatch, seq, qbit, metric, unit, workload):
     if rank != 0:
         return   # the CPU arm is a single process using the host cores; other ranks have no work
     world = int(os.environ.get('WORLD_SIZE', str(args.gpus)))
-    res = cpu_sample(spec, ubatch, seq, unit, max_steps=max(2, args.steps), budget_s=120.0)
+    res = cpu_sample(spec, ubatch, seq, unit, args.steps)
+    if args.dump_outputs:
+        dump_output(args.dump_outputs, 'logits', res['logits'])
     print(json.dumps({
         'impl': 'reference', 'metric': metric, 'value': res['value'], 'unit': unit, 'n_gpus': args.gpus,
         'steps': res['steps'], 'warmup': args.warmup, 'ms_per_step': res['seconds'] / res['steps'] * 1e3,
@@ -550,6 +567,8 @@ def run_gpu(args, spec, ubatch, seq, qbit, metric, unit, workload):
             checksum = None
             if rank == 0:
                 checksum = float(sum(t.double().abs().sum() for t in got[:N_INPUTS]))
+                if args.dump_outputs:
+                    dump_output(args.dump_outputs, 'logits', got[-1])
             run_phase(warmup, True)
             e2e_wall, _ = run_phase(steps, True)
             e2e_wall = allmax(e2e_wall) if world > 1 else e2e_wall
@@ -632,10 +651,12 @@ def run_quick(args, spec, ubatch, seq):
         start, end = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         start.record(stream)
         for i in range(args.steps):
-            shard(xs[i % 4])
+            logits = shard(xs[i % 4])
         end.record(stream)
         torch.cuda.synchronize()
     ms = start.elapsed_time(end)
+    if args.dump_outputs:
+        dump_output(args.dump_outputs, 'logits', logits)
     print(json.dumps({'quick': True, 'value': args.steps * ubatch / (ms * 1e-3), 'ms_per_step': ms / args.steps,
                       'gpu_launches': int(ops.launch_count() - l0)}))
 
@@ -644,7 +665,7 @@ def main():
     faulthandler.enable()   # a native crash in any thread prints every thread's Python stack to stderr
     ap = argparse.ArgumentParser()
     ap.add_argument('--gpus', type=int, default=1)
-    ap.add_argument('--steps', type=int, default=300)
+    ap.add_argument('--steps', type=int, default=None, help='timed micro-batches (default 300; 24 with --impl reference)')
     ap.add_argument('--warmup', type=int, default=20)
     ap.add_argument('--impl', choices=['ours', 'reference'], default='ours')
     ap.add_argument('--workload', choices=sorted(WORKLOADS), default='vit-base')
@@ -652,13 +673,16 @@ def main():
     ap.add_argument('--no-cpu-baseline', action='store_true')
     ap.add_argument('--quick', action='store_true', help='only a resident-input loop of direct shard calls (for ncu runs)')
     ap.add_argument('--eager', action='store_true', help='with --quick: no CUDA graph (every kernel visible to ncu)')
+    ap.add_argument('--dump-outputs', metavar='DIR', help="write the timed path's last outputs as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps is None:
+        args.steps = 24 if args.impl == 'reference' else 300   # a bounded CPU sample by default
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
     model, ubatch, seq, qbit, metric, unit = WORKLOADS[args.workload]
     ubatch = args.ubatch or ubatch
     spec = MODEL_SPECS[model]
     if args.impl == 'reference':
-        if args.steps == 300:
-            args.steps = 24   # a bounded CPU sample by default
         run_reference_arm(args, spec, ubatch, seq, qbit, metric, unit, args.workload)
         return
     if not torch.cuda.is_available():

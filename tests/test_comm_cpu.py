@@ -20,9 +20,12 @@ def _env(port):
     os.environ['CUDA_VISIBLE_DEVICES'] = ''   # this suite is the Gloo path
 
 
-def test_context_lifecycle_world1():
+def test_context_lifecycle_world1(monkeypatch):
     from pipeedge_b200.comm.p2p import DistP2pContext
-    _env(_free_port())
+    # This test runs in the pytest process: hiding the GPUs here (as `_env` does in the spawned ranks) would leave CUDA
+    # initialised without devices for every test after it. A world of one has no data plane, so it needs no hiding.
+    monkeypatch.setenv('MASTER_ADDR', '127.0.0.1')
+    monkeypatch.setenv('MASTER_PORT', str(_free_port()))
     ctx = DistP2pContext(('gloo',), {'world_size': 1, 'rank': 0}, lambda cmd, tensors: None)
     ctx.init()
     ctx.shutdown()

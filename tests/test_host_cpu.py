@@ -148,15 +148,24 @@ def test_product_never_imports_the_oracle():
     assert '/root/reference' not in src
 
 
-def test_bench_reference_arm_cli():
-    """`bench.py --impl reference` prints one JSON line with the contract's keys (tiny sample)."""
+def test_bench_reference_arm_cli(tmp_path):
+    """`bench.py --impl reference` prints one JSON line with the contract's keys (tiny sample), times exactly `--steps`
+    forwards, and `--dump-outputs` writes the last forward's logits: the oracle's logits for the seeded input."""
     import json
     out = subprocess.run([sys.executable, os.path.join(ROOT, 'bench.py'), '--impl', 'reference', '--steps', '1',
-                          '--warmup', '1'], capture_output=True, text=True, timeout=600, check=True)
+                          '--warmup', '1', '--dump-outputs', str(tmp_path)], capture_output=True, text=True, timeout=600,
+                         check=True)
     line = json.loads(out.stdout.strip().splitlines()[-1])
     assert line['impl'] == 'reference' and line['unit'] == 'images/s' and line['higher_is_better'] is True
     assert line['cpu_baseline']['kind'] == 'port' and line['e2e']['h2d_bytes_per_step'] == 0
-    assert line['value'] > 0
+    assert line['value'] > 0 and line['steps'] == 1
+    from oracle import shards as osh
+    from pipeedge_b200.synth import MODEL_SPECS, synth_input, synth_weights
+    spec = MODEL_SPECS['google/vit-base-patch16-224']
+    want = osh.shard_forward(spec, synth_weights(spec, seed=0), 1, spec.layers, synth_input(spec, 8, seed=1)).numpy()
+    got = np.load(tmp_path / 'logits.npy')
+    assert got.dtype == np.float32 and got.shape == (8, 1000)
+    np.testing.assert_allclose(got, want, rtol=1e-4, atol=1e-4)
 
 
 def _gemm_plan(m, n, k, epi):
